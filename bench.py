@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline metric of BASELINE.json: utterances/s (2 s @ 16 kHz) embedding extraction; PLDA scores/s.
 
-    python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--workload NAME] [--no-configs]
+    python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--workload NAME] [--no-configs] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path (fbank -> CMN -> model forward) over one batch of synthetic utterances per GPU.
@@ -567,7 +567,13 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the per-config legs (configs block)")
     ap.add_argument("--sustained-s", type=float, default=2.0, help="length of the seconds-long sustained leg (0 = skip)")
     ap.add_argument("--tc-version", type=int, default=0, help="override the engine's tcgen05 kernel generation (1,2,3)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the embeddings of the last timed step (rank 0's batch) to DIR/embeddings.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's embeddings; it cannot be combined with --impl reference")
     wl = args.workload
     if args.impl == "reference":
         run_reference(args, wl)
@@ -607,8 +613,11 @@ def main():
     embed_dim = model.embed_dim
 
     # ---------------- device-resident throughput (`value`): K steps + the one all-gather, best of 3 windows
+    last_step = []
+
     def value_run():
         local_embs = [model.extract_from_wav(wav_dev[i % nrot]) for i in range(args.steps)]
+        last_step[:] = local_embs[-1:]
         allemb = torch.cat(local_embs, 0)
         return parallel.gather_embeddings(allemb, allemb.shape[0] * world)  # the one NCCL all-gather of the job
     if sampler:
@@ -620,6 +629,11 @@ def main():
         clocks = sampler.read() if sampler.nvml is not None else None
     assert gathered.shape[0] == args.steps * B * world and torch.isfinite(gathered).all()
     value = world * B * args.steps / (ms_total * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # inputs and weights are seeded (make_wavs seed 100 + rank, from_synthetic seed 0): two builds of the project run
+        # with the same arguments can be compared output for output
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "embeddings.npy"), last_step[0].float().cpu().numpy())
 
     # ---------------- end-to-end through the public host-buffer API (`e2e`)
     # B200SpeakerModel.extract_stream: every step copies that step's pinned int16 PCM batch H2D, runs fbank+CMN+forward

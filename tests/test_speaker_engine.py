@@ -144,3 +144,37 @@ def test_cpp_seam_reference_engine_with_b200_model(nsamp, chunk, tmp_path):
     rel = np.linalg.norm(emb - want) / np.linalg.norm(want)
     print(f"C++ seam nsamp {nsamp} chunk {chunk}: rel {rel:.2e}")
     assert rel < 1e-4
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("nsamp,chunk", [(50000, 32000), (9000, 32000), (50000, 0)])
+def test_cpp_b200_speaker_model_per_chunk_matches_oracle(nsamp, chunk, tmp_path):
+    """wespeaker::B200SpeakerModel (csrc/runtime/b200_speaker_model.cc, in build/libb200_model_harness.so) called through
+    the virtual SpeakerModel::ExtractEmbedding, one chunk per call, with no file from outside this repository: the
+    reference's native fbank frames of this PCM (fixture) are chunked and mean-normalised by the Python restatement (pinned
+    above on the reference's own outputs) on both sides, and the average of the B200 embeddings is compared with the CPU
+    oracle model's.  The interface is a stand-in (oracle/seam_shim), so compatibility with the real speaker_model.h is not
+    checked here; test_cpp_seam_reference_engine_with_b200_model does that where the WeSpeaker sources were built."""
+    import ctypes as C
+    import os
+    from wespeaker_b200.models import from_synthetic
+    so = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "build", "libb200_model_harness.so")
+    name = "ECAPA_TDNN_c512"
+    m = from_synthetic(name, 0, precision="fp32")
+    flat = str(tmp_path / "model.wsb")
+    m.export_flat(flat)
+    L = C.CDLL(so)
+    L.b200_model_extract_chunks.restype = C.c_int
+    L.b200_model_extract_chunks.argtypes = [C.c_char_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int]
+    frames = list(G_REF[f"full_{nsamp}"])                      # the reference's native fbank frames of this PCM
+    chunks = np.ascontiguousarray(np.stack([ref.apply_mean(c) for c in ref.extract_feature(frames, chunk)]))
+    embs = np.zeros((chunks.shape[0], 192), dtype=np.float32)
+    assert L.b200_model_extract_chunks(flat.encode(), 0, chunks.ctypes.data, chunks.shape[0], chunks.shape[1],
+                                       chunks.shape[2], embs.ctypes.data, 192) == 0
+    emb = embs.sum(axis=0) / chunks.shape[0]
+    sd = syn.make_state_dict(name, seed=0)
+    fwd = lambda feats: models_torch.forward(name, sd, torch.as_tensor(feats, dtype=torch.float32))
+    want = ref.extract_embedding(frames, chunk, lambda c: fwd(c[None])[0].numpy())
+    rel = np.linalg.norm(emb - want) / np.linalg.norm(want)
+    print(f"B200SpeakerModel per chunk, nsamp {nsamp} chunk {chunk}: rel {rel:.2e}")
+    assert rel < 1e-4
